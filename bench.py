@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Mpixels/s of baseline 4:2:0 batch decode on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload hd1024|uhd]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload hd1024|uhd] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path (prescan -> entropy -> stitch -> fused IDCT+colour) over
 one batch of synthetic JPEGs.  N=1 workload = BASELINE.json configs[1]: 1024 x 1920x1080
@@ -9,7 +9,8 @@ one batch of synthetic JPEGs.  N=1 workload = BASELINE.json configs[1]: 1024 x 1
 and pixels left in HBM; `e2e` = the same metric through the public C ABI with pinned HOST
 buffers on both sides (header parse + H2D + kernels + D2H inside the timed region).
 `--impl reference` times the unmodified reference (oracle/_ref, SSE2 build) on all host cores.
-One JSON line on stdout (rank 0).
+One JSON line on stdout (rank 0).  `--dump-outputs DIR` also writes what the last timed step decoded (rank 0's batch) as
+.npy files, so that two builds can be compared output for output: the inputs are the same seeded images on every run.
 """
 import argparse
 import ctypes as C
@@ -24,6 +25,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree it runs from as it found it
 
 WORKLOADS = {
     # name: (n_images, w, h, quality, pixel_type_name, algorithmic bytes per source pixel for the fused kernel)
@@ -238,6 +240,31 @@ def cpu_reference_run(wl, jpegs, pixel_type, n_sample, threads, passes=3):
     return mp / best, best
 
 
+def dump_outputs(out_dir, b, st, n_img, oh0, row_bytes):
+    """The last timed step's results as a caller of the batch would read them: per image its status and the CRC-32 of its
+    pixels (rows x bytes that hold image pixels), and the pixel bytes of a fixed seeded sample of up to 8 images at a fixed
+    seeded sample of up to 2^20 byte offsets.  float64 / float32 .npy files, about 40 MB at most."""
+    import zlib
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    img_bytes = oh0 * row_bytes
+    pick = np.sort(rng.choice(n_img, size=min(8, n_img), replace=False))
+    offs = np.sort(rng.choice(img_bytes, size=min(1 << 20, img_bytes), replace=False))
+    crc = np.zeros(n_img, dtype=np.float64)
+    pixels = np.zeros((len(pick), len(offs)), dtype=np.float32)
+    for i in range(n_img):
+        img = np.ascontiguousarray(b.read_output(i)[:oh0, :row_bytes]).reshape(-1)
+        crc[i] = zlib.crc32(img)
+        k = np.searchsorted(pick, i)
+        if k < len(pick) and pick[k] == i:
+            pixels[k] = img[offs]
+    np.save(os.path.join(out_dir, "status.npy"), np.asarray(st, dtype=np.float64))
+    np.save(os.path.join(out_dir, "crc32.npy"), crc)
+    np.save(os.path.join(out_dir, "pixels.npy"), pixels)
+    np.save(os.path.join(out_dir, "pixel_images.npy"), pick.astype(np.float64))
+    np.save(os.path.join(out_dir, "pixel_offsets.npy"), offs.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -250,13 +277,18 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--pipelined", action="store_true", help="also time the steps with two resident batches in flight")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's decoded outputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     W = max(args.warmup, 0)
-    K = max(args.steps, 1)
+    K = args.steps
     cpu_facts = host_cpu_facts()
     threads = cpu_facts["usable"]
     n_img = args.images if args.images > 0 else wl["n"]
@@ -371,7 +403,7 @@ def main():
     dev_ms, stage = 0.0, {k: 0.0 for k in J.TIMING_NAMES}
     launches = 0
     for _ in range(K):
-        b.decode(J.JPEGB200_OUT_DEVICE); b.download(); b.wait()
+        b.decode(J.JPEGB200_OUT_DEVICE); b.download(); st = b.wait()
         tm = b.timings()
         dev_ms += tm["total"]
         for k in stage:
@@ -386,6 +418,11 @@ def main():
     value = world * mp_per_step_rank / (ms_step / 1e3)
     idct_ms = stage["idct"] / K
     entropy_ms = stage["entropy"] / K
+    sh0 = {2: 1, 4: 2, 8: 3}.get(opt & 14, 0)
+    ow0, oh0 = (wl["w"] + (1 << sh0) - 1) >> sh0, (wl["h"] + (1 << sh0) - 1) >> sh0
+    row_bytes = (ow0 * J.bits_per_pixel(pixel_type) + 7) // 8     # bytes of a row that hold image pixels (dithered rows are MCU-padded)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, b, st, n_img, oh0, row_bytes)
 
     # ---- the same steps with TWO batches in flight (informational): step k+1's entropy kernel (latency bound, ~45 % of
     # the issue slots) runs beside step k's IDCT kernel on another stream.  Wall clock around 2K decodes, max over ranks. ----
@@ -428,9 +465,6 @@ def main():
         return (img if rc == 1 else None), "C restatement (oracle/jpegdec_oracle.c)"
 
     parity, parity_all = None, None
-    sh0 = {2: 1, 4: 2, 8: 3}.get(opt & 14, 0)
-    ow0, oh0 = (wl["w"] + (1 << sh0) - 1) >> sh0, (wl["h"] + (1 << sh0) - 1) >> sh0
-    row_bytes = (ow0 * J.bits_per_pixel(pixel_type) + 7) // 8     # bytes of a row that hold image pixels (dithered rows are MCU-padded)
     try:
         if rank == 0:
             nchk = min(4, unique)

@@ -26,6 +26,23 @@ def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()[:16]
 
 
+def log_sha(log):
+    """digest of a draw-callback log (a list of equal-length integer tuples)"""
+    return sha(np.asarray(log, dtype=np.int64))
+
+
+def reference_calls(name):
+    """What the compiled reference returned for the calls one test compares with: {case key: record of digests}
+    (tests/golden/reference/<name>.json, written by tests/golden/make_reference_golden.py)."""
+    return json.load(open(os.path.join(GOLD, "reference", name + ".json")))
+
+
+def check_input(rec, data, what):
+    """synthetic inputs are re-encoded at test time: they must be the bytes the golden record was made from"""
+    assert sha(np.frombuffer(data, dtype=np.uint8)) == rec["input"], \
+        "%s: synthetic JPEG differs from the one the reference was run on (Pillow / OpenCV encoder changed?)" % (what,)
+
+
 def bpp_of(pt):
     return {0: 16, 1: 16, 2: 32, 3: 8, 4: 4, 5: 2, 6: 1}[pt]
 

@@ -6,7 +6,7 @@ import hashlib, json, os, subprocess, sys, tempfile
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-from tests.c_api import build_reference_examples as B
+from oracle import ref_examples as B
 
 FIXTURES = ["tulips", "croptest", "ncc1701", "sciopero", "batman"]
 

@@ -60,9 +60,9 @@ def test_c_and_cpp_callers_match_reference(tmp_path):
 
 # ---- the reference's own programs, unmodified (SURVEY.md 8(f)3) ----
 def _ref_examples():
-    """Binaries built by tests/c_api/build_reference_examples.py.  Built here when the reference sources are present
-    (this container); on the GPU box the prebuilt files travel with the snapshot."""
-    from tests.c_api import build_reference_examples as B
+    """Binaries built by oracle/ref_examples.py into oracle/_ref/examples.  Built here when the reference sources are present;
+    elsewhere the ones build() made where they were present are used."""
+    from oracle import ref_examples as B
     if B.available():
         B.build()
     names = ["ref_c_cmdline", "ref_perf_test", "ref_jpegdec_test"]
@@ -71,7 +71,7 @@ def _ref_examples():
 
 
 def test_reference_programs_compile_unmodified_against_this_library():
-    from tests.c_api import build_reference_examples as B
+    from oracle import ref_examples as B
     if not B.available():
         pytest.skip("reference sources not on this machine")
     ex = _ref_examples()
@@ -90,7 +90,7 @@ def test_reference_programs_run_on_the_gpu_and_match_the_reference_build(tmp_pat
     import json
     ex = _ref_examples()
     if ex is None:
-        pytest.skip("prebuilt reference programs not present (build them where /root/reference exists)")
+        pytest.skip("reference programs not built (build() makes them where the reference sources exist)")
     gold = json.load(open(os.path.join(T.GOLD, "ref_examples.json")))["fixtures"]
     for name, g in gold.items():
         bmp = str(tmp_path / (name + ".bmp"))

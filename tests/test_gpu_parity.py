@@ -1,5 +1,6 @@
 """GPU tier (-m gpu): parity of the CUDA path, called through the C ABI, against the compiled reference
-(oracle/_ref, travels with the snapshot), the C restatement and the committed digests.  Bit-exact."""
+(oracle/_ref where it was built, and what it returned as recorded in tests/golden/reference/), the C restatement and the
+committed digests.  Bit-exact."""
 import ctypes as C
 import hashlib
 import json
@@ -118,21 +119,37 @@ def _collect(j, pt, options, x=0, y=0):
     return draw, log, blocks
 
 
+CALLBACK_CASES = [("sciopero", 0, 0, 10, 20, 0), ("sciopero", 2, 0, 0, 0, 0), ("sciopero", 3, 0, 0, 0, 0),
+                  ("sciopero", 0, 2, 0, 0, 0), ("sciopero", 0, 4, 3, 5, 0), ("sciopero", 0, 8, 0, 0, 0),
+                  ("tulips", 0, 0, 0, 0, 0), ("tulips", 0, J.JPEG_USES_DMA, 0, 0, 0), ("tulips", 0, 0, 0, 0, 3),
+                  ("ncc1701", 2, 0, 0, 0, 0), ("zebra", 1, 0, 0, 0, 0), ("zebra", 0, 2, 0, 0, 0), ("lange", 3, 4, 0, 0, 0),
+                  ("tulips", 0, J.JPEG_LUMA_ONLY, 0, 0, 0)]
+
+
+def _callback_key(mode, case):
+    return "%s/%s/%d/%d/%d/%d/%d" % ((mode,) + case)
+
+
+def record_callbacks(refs):
+    out = {}
+    for mode, arith in MODES:
+        for case in CALLBACK_CASES:
+            name, pt, opt, xo, yo, maxm = case
+            rc_r, err_r, img_r, log_r = refs[mode].decode_cb(T.image(name), pt, opt, xoff=xo, yoff=yo, max_mcus=maxm)
+            out[_callback_key(mode, case)] = {"rc": rc_r, "log": T.log_sha([r[:6] for r in log_r]), "shape": list(img_r.shape),
+                                              "sha": T.sha(img_r)}
+    return out
+
+
 @pytest.mark.parametrize("mode,arith", MODES)
 def test_single_image_api_callbacks_match_reference(mode, arith):
     """JPEG_openRAM -> setPixelType -> decode: same callback sequence (x, y, iWidth, iHeight, iWidthUsed, iBpp)
     and same delivered pixels as the reference, incl. decode offset, JPEG_USES_DMA and setMaxOutputSize."""
-    ref = _ref(mode)
-    if ref is None:
-        pytest.skip("oracle/_ref not present")
-    cases = [("sciopero", 0, 0, 10, 20, 0), ("sciopero", 2, 0, 0, 0, 0), ("sciopero", 3, 0, 0, 0, 0),
-             ("sciopero", 0, 2, 0, 0, 0), ("sciopero", 0, 4, 3, 5, 0), ("sciopero", 0, 8, 0, 0, 0),
-             ("tulips", 0, 0, 0, 0, 0), ("tulips", 0, J.JPEG_USES_DMA, 0, 0, 0), ("tulips", 0, 0, 0, 0, 3),
-             ("ncc1701", 2, 0, 0, 0, 0), ("zebra", 1, 0, 0, 0, 0), ("zebra", 0, 2, 0, 0, 0), ("lange", 3, 4, 0, 0, 0),
-             ("tulips", 0, J.JPEG_LUMA_ONLY, 0, 0, 0)]
-    for name, pt, opt, xo, yo, maxm in cases:
+    want = T.reference_calls("gpu_callbacks")
+    for case in CALLBACK_CASES:
+        name, pt, opt, xo, yo, maxm = case
+        g = want[_callback_key(mode, case)]
         data = T.image(name)
-        rc_r, err_r, img_r, log_r = ref.decode_cb(data, pt, opt, xoff=xo, yoff=yo, max_mcus=maxm)
         j = J.JPEGDEC()
         draw, log, blocks = _collect(j, pt, opt)
         assert j.openRAM(data, draw) == 1
@@ -141,83 +158,95 @@ def test_single_image_api_callbacks_match_reference(mode, arith):
         if maxm:
             j.setMaxOutputSize(maxm)
         rc = j.decode(xo, yo, opt)
-        assert rc == rc_r == 1, (name, pt, opt, j.getLastError())
-        assert [l for l in log] == [tuple(r[:6]) for r in log_r], (name, pt, opt)
+        assert rc == g["rc"] == 1, (name, pt, opt, j.getLastError())
+        assert T.log_sha(log) == g["log"], (name, pt, opt)
         # assemble the tight image from the delivered blocks
-        out = np.zeros_like(img_r)
+        out = np.zeros(g["shape"], np.uint8)
         for (x, y, w, h, wu, bpp), buf in zip(log, blocks):
             pitch = (w * bpp + 7) // 8
             a = np.frombuffer(buf, dtype=np.uint8).reshape(h, pitch)
             bw = wu * bpp // 8
             x0 = (x - xo) * bpp // 8
             out[y - yo:y - yo + h, x0:x0 + bw] = a[:, :bw]
-        assert np.array_equal(out, img_r), (name, pt, opt)
+        assert T.sha(out) == g["sha"], (name, pt, opt)
         j.close()
+
+
+# framebuffer mode: tulips has a multiple-of-16 width (reference pitch = image width, identical bytes); the others have a
+# width / height that is not a multiple of the MCU: the reference's SSE2 build stores whole MCUs (the right edge runs on into
+# the next line), its scalar build clips -- the visible w x h region must match either way
+FRAMEBUFFER_CASES = [("tulips", 640, 480, pt) for pt in (0, 2, 3)] + \
+    [(name, w, h, pt) for name, w, h in (("sciopero", 300, 300), ("ncc1701", 240, 77), ("zebra", 320, 240)) for pt in (0, 2)]
+
+
+def record_framebuffer_crop_thumb_dither(refs):
+    out = {}
+    for mode, arith in MODES:
+        ref = refs[mode]
+        for name, w, h, pt in FRAMEBUFFER_CASES:
+            rc_r, err_r, fb_r = ref.decode_fb(T.image(name), pt, 0)
+            n = w * h * T.bpp_of(pt) // 8
+            out["%s/fb/%s/%d" % (mode, name, pt)] = {"rc": rc_r, "bytes": int(fb_r.size), "sha": T.sha(fb_r[:n])}
+        rc_r, err_r, img_r, log_r = ref.decode_cb(T.image("tulips"), 0, 0, crop=(50, 50, 125, 170))
+        out[mode + "/crop"] = {"rc": rc_r, "log": T.log_sha([r[:6] for r in log_r]), "sha": T.sha(img_r[:176, :256])}
+        rc_r, err_r, img_r, log_r = ref.decode_cb(T.image("thumb_test"), 0, J.JPEG_EXIF_THUMBNAIL)
+        out[mode + "/thumb"] = {"rc": rc_r, "log": T.log_sha([r[:6] for r in log_r]), "shape": list(img_r.shape), "sha": T.sha(img_r)}
+        rc_r, err_r, img_r, log_r = ref.decode_dither(T.image("zebra"), J.ONE_BIT_DITHERED, 0)
+        out[mode + "/dither"] = {"rc": rc_r, "log": T.log_sha([r[:6] for r in log_r]), "shape": list(img_r.shape),
+                                 "sha": T.sha(img_r[:, :40])}
+    return out
 
 
 @pytest.mark.parametrize("mode,arith", MODES)
 def test_single_image_api_framebuffer_crop_thumb_dither(mode, arith):
-    ref = _ref(mode)
-    if ref is None:
-        pytest.skip("oracle/_ref not present")
-    # framebuffer mode, multiple-of-16 width: identical bytes (reference pitch = image width)
-    data = T.image("tulips")
-    for pt in (0, 2, 3):
-        rc_r, err_r, fb_r = ref.decode_fb(data, pt, 0)
-        j = J.JPEGDEC(); assert j.openRAM(data); j.setArithMode(arith); j.setPixelType(pt)
-        fb = np.zeros_like(fb_r); j.setFramebuffer(fb)
-        assert j.decode(0, 0, 0) == rc_r == 1
-        n = 640 * 480 * T.bpp_of(pt) // 8
-        assert np.array_equal(fb[:n], fb_r[:n])
-    # framebuffer mode, width / height not multiples of the MCU: the reference's SSE2 build stores whole MCUs (the right
-    # edge runs on into the next line), its scalar build clips -- the visible w x h region must match either way
-    for name, w, h in (("sciopero", 300, 300), ("ncc1701", 240, 77), ("zebra", 320, 240)):
+    want = T.reference_calls("gpu_framebuffer_crop_thumb_dither")
+    for name, w, h, pt in FRAMEBUFFER_CASES:
+        g = want["%s/fb/%s/%d" % (mode, name, pt)]
         d2 = T.image(name)
-        for pt in (0, 2):
-            rc_r, err_r, fb_r = ref.decode_fb(d2, pt, 0)
-            j = J.JPEGDEC(); assert j.openRAM(d2); j.setArithMode(arith); j.setPixelType(pt)
-            fb = np.zeros_like(fb_r); j.setFramebuffer(fb)
-            assert j.decode(0, 0, 0) == rc_r == 1
-            n = w * h * T.bpp_of(pt) // 8
-            assert np.array_equal(fb[:n], fb_r[:n]), (name, pt, mode)
+        j = J.JPEGDEC(); assert j.openRAM(d2); j.setArithMode(arith); j.setPixelType(pt)
+        fb = np.zeros(g["bytes"], np.uint8); j.setFramebuffer(fb)
+        assert j.decode(0, 0, 0) == g["rc"] == 1
+        n = w * h * T.bpp_of(pt) // 8
+        assert T.sha(fb[:n]) == g["sha"], (name, pt, mode)
     # crop through callbacks (reference test 2): exactly the snapped rectangle, same pixels
-    rc_r, err_r, img_r, log_r = ref.decode_cb(data, 0, 0, crop=(50, 50, 125, 170))
+    data = T.image("tulips")
+    g = want[mode + "/crop"]
     j = J.JPEGDEC(); draw, log, blocks = _collect(j, 0, 0)
     assert j.openRAM(data, draw); j.setArithMode(arith); j.setCropArea(50, 50, 125, 170)
     assert j.decode(0, 0, 0) == 1
-    assert log == [tuple(r[:6]) for r in log_r]
+    assert T.log_sha(log) == g["log"]
     out = np.zeros((176, 256), np.uint8)
     for (x, y, w, h, wu, bpp), buf in zip(log, blocks):
         a = np.frombuffer(buf, dtype=np.uint8).reshape(h, w * 2)
         out[y:y + h, x * 2:(x + wu) * 2] = a[:, :wu * 2]
-    assert np.array_equal(out, img_r[:176, :256])
+    assert T.sha(out) == g["sha"]
     # EXIF thumbnail (reference test 10): 320x240
     tdata = T.image("thumb_test")
-    rc_r, err_r, img_r, log_r = ref.decode_cb(tdata, 0, J.JPEG_EXIF_THUMBNAIL)
+    g = want[mode + "/thumb"]
     j = J.JPEGDEC(); draw, log, blocks = _collect(j, 0, 0)
     assert j.openRAM(tdata, draw) and j.hasThumb() and (j.getThumbWidth(), j.getThumbHeight()) == (320, 240)
     j.setArithMode(arith)
-    assert j.decode(0, 0, J.JPEG_EXIF_THUMBNAIL) == rc_r == 1
+    assert j.decode(0, 0, J.JPEG_EXIF_THUMBNAIL) == g["rc"] == 1
     assert (j.getWidth(), j.getHeight()) == (320, 240)
-    assert log == [tuple(r[:6]) for r in log_r]
-    out = np.zeros_like(img_r)
+    assert T.log_sha(log) == g["log"]
+    out = np.zeros(g["shape"], np.uint8)
     for (x, y, w, h, wu, bpp), buf in zip(log, blocks):
         a = np.frombuffer(buf, dtype=np.uint8).reshape(h, w * 2)
         out[y:y + h, x * 2:(x + wu) * 2] = a[:, :wu * 2]
-    assert np.array_equal(out, img_r)
+    assert T.sha(out) == g["sha"]
     # decodeDither through the callback
     zdata = T.image("zebra")
-    rc_r, err_r, img_r, log_r = ref.decode_dither(zdata, J.ONE_BIT_DITHERED, 0)
+    g = want[mode + "/dither"]
     j = J.JPEGDEC(); draw, log, blocks = _collect(j, 6, 0)
     assert j.openRAM(zdata, draw); j.setArithMode(arith); j.setPixelType(J.ONE_BIT_DITHERED)
     dbuf = np.zeros((320 + 32) * 16, np.uint8)
-    assert j.decodeDither(dbuf, 0) == rc_r == 1
-    assert log == [tuple(r[:6]) for r in log_r]
-    out = np.zeros_like(img_r)
+    assert j.decodeDither(dbuf, 0) == g["rc"] == 1
+    assert T.log_sha(log) == g["log"]
+    out = np.zeros(g["shape"], np.uint8)
     for (x, y, w, h, wu, bpp), buf in zip(log, blocks):
         a = np.frombuffer(buf, dtype=np.uint8).reshape(h, (w + 7) // 8)
         out[y:y + h, :(wu + 7) // 8] = a[:, :(wu + 7) // 8]
-    assert np.array_equal(out[:, :40], img_r[:, :40])
+    assert T.sha(out[:, :40]) == g["sha"]
 
 
 def test_corrupt_inputs_do_not_poison_the_batch(ctxs):
@@ -372,10 +401,7 @@ def test_progressive_files_give_the_dc_thumbnail(ctxs):
         assert T.sha(out) == g[name]["sse/565le/opt0"]["sha"], name
 
 
-def test_seeded_random_sweep_on_the_gpu(ctxs):
-    """Seeded random 4:2:0 / 4:4:4 / 4:2:2 / gray files of random size and quality (15..100: every mix of the IDCT kernel's
-    block classes), random restart interval, decoded in mixed batches per pixel type at full size and 1/2, both arithmetic
-    modes, against the compiled reference."""
+def _gpu_sweep_files():
     rng = np.random.default_rng(77)
     files = []
     for case in range(48):
@@ -384,18 +410,39 @@ def test_seeded_random_sweep_on_the_gpu(ctxs):
         gray = bool(rng.integers(0, 6) == 0)
         sub = ["4:2:0", "4:2:0", "4:2:2", "4:4:4"][int(rng.integers(0, 4))]
         files.append((synth.synth_jpeg(w, h, 5000 + case, q, subsampling=sub, gray=gray, restart_rows=int(rng.integers(0, 3))), gray))
+    return files
+
+
+def record_gpu_sweep(refs):
+    files = _gpu_sweep_files()
+    out = {"input/%d" % i: {"input": T.sha(np.frombuffer(d, dtype=np.uint8))} for i, (d, g) in enumerate(files)}
     for mode, arith in MODES:
-        ref = _ref(mode)
-        if ref is None:
-            pytest.skip("oracle/_ref not present")
         for pt in (0, 2, 3):
             for opt in (0, 2):
-                use = [d for d, g in files if not (g and pt == 2)]
-                outs, st, tim, cnt = J.decode_batch_to_host(ctxs[arith], use, pt, opt)
+                for i, (d, gray) in enumerate(files):
+                    if not (gray and pt == 2):
+                        rc, err, img, _ = refs[mode].decode_cb(d, pt, opt, want_log=False)
+                        out["%s/%d/%d/%d" % (mode, pt, opt, i)] = {"rc": rc, "shape": list(img.shape), "sha": T.sha(img)}
+    return out
+
+
+def test_seeded_random_sweep_on_the_gpu(ctxs):
+    """Seeded random 4:2:0 / 4:4:4 / 4:2:2 / gray files of random size and quality (15..100: every mix of the IDCT kernel's
+    block classes), random restart interval, decoded in mixed batches per pixel type at full size and 1/2, both arithmetic
+    modes, against what the compiled reference returned for them."""
+    files = _gpu_sweep_files()
+    want = T.reference_calls("gpu_sweep")
+    for i, (d, gray) in enumerate(files):
+        T.check_input(want["input/%d" % i], d, i)
+    for mode, arith in MODES:
+        for pt in (0, 2, 3):
+            for opt in (0, 2):
+                use = [i for i, (d, g) in enumerate(files) if not (g and pt == 2)]
+                outs, st, tim, cnt = J.decode_batch_to_host(ctxs[arith], [files[i][0] for i in use], pt, opt)
                 assert st == [0] * len(use)
-                for k, (d, o) in enumerate(zip(use, outs)):
-                    rc, err, img, _ = ref.decode_cb(d, pt, opt, want_log=False)
-                    assert rc == 1 and np.array_equal(o, img), (k, mode, pt, opt)
+                for k, (i, o) in enumerate(zip(use, outs)):
+                    g = want["%s/%d/%d/%d" % (mode, pt, opt, i)]
+                    assert g["rc"] == 1 and list(o.shape) == g["shape"] and T.sha(o) == g["sha"], (k, mode, pt, opt)
 
 
 def test_pipeline_switches_give_the_default_result():
@@ -563,52 +610,92 @@ def test_two_threads_two_contexts(ctxs):
     assert not errs, errs
 
 
+CROP_SCALE_CASES = [(name, crop, pt, opt)
+                    for name, crops in (("tulips", [(96, 64, 256, 192), (50, 50, 125, 170), (0, 0, 64, 64)]), ("zebra", [(32, 16, 128, 96)]))
+                    for crop in crops for pt in (0, 2, 3) for opt in (0, 2, 4, 8)]
+
+
+def _crop_scale_key(mode, name, crop, pt, opt):
+    return "%s/%s/%s/%d/%d" % (mode, name, ",".join(map(str, crop)), pt, opt)
+
+
+def _crop_geometry(j, opt):
+    """(snapped crop x, scaled width of the MCU-aligned image)"""
+    cx, cy, cw, ch = j.getCropArea()
+    sh = {0: 0, 2: 1, 4: 2, 8: 3}[opt]
+    mcu_w = (16 if j.getSubSample() in (0x21, 0x22) else 8) >> sh
+    return cx, -(-j.getWidth() // (mcu_w << sh)) * mcu_w
+
+
+def _crop_groups(log, cx, aligned_w, shape):
+    """per callback: (rows of the image it covers, byte offset, bytes it wrote, bytes it spans); None when it places nothing.
+    A group that reaches the image's right edge before it is full carries stale bytes in the reference (never written) beyond
+    the last MCU it placed: only the written part is compared."""
+    for (x, y, w, h, wu, bpp) in log:
+        written = min(wu, aligned_w - (cx + x))
+        bw, x0 = written * bpp // 8, x * bpp // 8
+        ys = slice(max(y, 0), min(y + h, shape[0]))
+        if x0 < 0 or ys.start >= ys.stop or bw <= 0:
+            yield None
+        else:
+            yield ys, x0, bw, wu * bpp // 8
+
+
+def record_crop_scale(refs):
+    out = {}
+    for mode, arith in MODES:
+        for name, crop, pt, opt in CROP_SCALE_CASES:
+            data = T.image(name)
+            rc_r, err_r, img_r, log_r = refs[mode].decode_cb(data, pt, opt, crop=crop)
+            log = [tuple(r[:6]) for r in log_r]
+            j = J.JPEGDEC(); assert j.openRAM(data); j.setPixelType(pt); j.setCropArea(*crop)
+            cx, aligned_w = _crop_geometry(j, opt)
+            cx, cy, cw, ch = j.getCropArea()
+            j.close()
+            want = img_r.copy()
+            for grp in _crop_groups(log, cx, aligned_w, img_r.shape):
+                if grp is not None:
+                    ys, x0, bw, span = grp
+                    want[ys, x0 + bw:x0 + span] = 0
+            rec = {"rc": rc_r, "log": T.log_sha(log), "shape": list(img_r.shape), "sha": T.sha(want)}
+            if opt == 0:
+                rec["framebuffer"] = T.sha(img_r[:ch, :cw * T.bpp_of(pt) // 8])
+            out[_crop_scale_key(mode, name, crop, pt, opt)] = rec
+    return out
+
+
 @pytest.mark.parametrize("mode,arith", MODES)
 def test_crop_times_scale_callbacks_and_framebuffer(mode, arith):
     """setCropArea combined with 1/2, 1/4, 1/8 (SURVEY.md A.5: the reference compares scaled MCU positions with the unscaled
-    crop rectangle) through the callback and into a framebuffer: same callback sequence, same pixels as the live reference
+    crop rectangle) through the callback and into a framebuffer: same callback sequence, same pixels as the reference
     (src/jpeg.inl:5111-5137, :5114-5124); the geometry alone is pinned on the CPU in tests/test_host.py."""
-    ref = _ref(mode)
-    if ref is None:
-        pytest.skip("oracle/_ref not present")
-    for name, crops in (("tulips", [(96, 64, 256, 192), (50, 50, 125, 170), (0, 0, 64, 64)]), ("zebra", [(32, 16, 128, 96)])):
+    want = T.reference_calls("gpu_crop_scale")
+    for name, crop, pt, opt in CROP_SCALE_CASES:
         data = T.image(name)
-        for crop in crops:
-            for pt in (0, 2, 3):
-                for opt in (0, 2, 4, 8):
-                    rc_r, err_r, img_r, log_r = ref.decode_cb(data, pt, opt, crop=crop)
-                    j = J.JPEGDEC(); draw, log, blocks = _collect(j, pt, opt)
-                    assert j.openRAM(data, draw); j.setArithMode(arith); j.setPixelType(pt); j.setCropArea(*crop)
-                    assert j.decode(0, 0, opt) == rc_r == 1
-                    assert log == [tuple(r[:6]) for r in log_r], (name, crop, pt, opt)
-                    out = np.zeros_like(img_r)
-                    want = img_r.copy()
-                    cx, cy, cw, ch = j.getCropArea()
-                    sh = {0: 0, 2: 1, 4: 2, 8: 3}[opt]
-                    mcu_w = (16 if j.getSubSample() in (0x21, 0x22) else 8) >> sh
-                    aligned_w = -(-j.getWidth() // (mcu_w << sh)) * mcu_w          # scaled width of the MCU-aligned image
-                    for (x, y, w, h, wu, bpp), buf in zip(log, blocks):
-                        a = np.frombuffer(buf, dtype=np.uint8).reshape(h, w * bpp // 8)
-                        # a group that reaches the image's right edge before it is full carries stale bytes in the reference
-                        # (never written) beyond the last MCU it placed: only the written part is compared
-                        written = min(wu, aligned_w - (cx + x))
-                        bw, x0 = written * bpp // 8, x * bpp // 8
-                        ys = slice(max(y, 0), min(y + h, out.shape[0]))
-                        if x0 < 0 or ys.start >= ys.stop or bw <= 0:
-                            continue
-                        out[ys, x0:x0 + bw] = a[ys.start - y:ys.stop - y, :bw][:, :out.shape[1] - x0]
-                        want[ys, x0 + bw:x0 + wu * bpp // 8] = 0
-                    assert np.array_equal(out, want), (name, crop, pt, opt)
-                    j.close()
-                    if opt == 0:
-                        # framebuffer + crop (pitch = crop width, :5116): the cropped image the callbacks deliver.  (The reference
-                        # itself clobbers the first pixels of most lines here: the one MCU its inclusive crop test lets through
-                        # past the right edge is stored beyond the pitch -- documented deviation, DESIGN.md.)
-                        j = J.JPEGDEC(); assert j.openRAM(data); j.setArithMode(arith); j.setPixelType(pt); j.setCropArea(*crop)
-                        cx, cy, cw, ch = j.getCropArea()
-                        bypp = T.bpp_of(pt) // 8
-                        fb = np.zeros((ch + 32) * cw * bypp, np.uint8); j.setFramebuffer(fb)
-                        assert j.decode(0, 0, opt) == 1
-                        got = fb[:ch * cw * bypp].reshape(ch, cw * bypp)
-                        assert np.array_equal(got, img_r[:ch, :cw * bypp]), (name, crop, pt, opt, "framebuffer")
-                        j.close()
+        g = want[_crop_scale_key(mode, name, crop, pt, opt)]
+        j = J.JPEGDEC(); draw, log, blocks = _collect(j, pt, opt)
+        assert j.openRAM(data, draw); j.setArithMode(arith); j.setPixelType(pt); j.setCropArea(*crop)
+        assert j.decode(0, 0, opt) == g["rc"] == 1
+        assert T.log_sha(log) == g["log"], (name, crop, pt, opt)
+        out = np.zeros(g["shape"], np.uint8)
+        cx, aligned_w = _crop_geometry(j, opt)
+        for grp, (x, y, w, h, wu, bpp), buf in zip(_crop_groups(log, cx, aligned_w, out.shape), log, blocks):
+            if grp is None:
+                continue
+            ys, x0, bw, span = grp
+            a = np.frombuffer(buf, dtype=np.uint8).reshape(h, w * bpp // 8)
+            out[ys, x0:x0 + bw] = a[ys.start - y:ys.stop - y, :bw][:, :out.shape[1] - x0]
+        assert T.sha(out) == g["sha"], (name, crop, pt, opt)
+        j.close()
+        if opt == 0:
+            # framebuffer + crop (pitch = crop width, :5116): the cropped image the callbacks deliver.  (The reference
+            # itself clobbers the first pixels of most lines here: the one MCU its inclusive crop test lets through
+            # past the right edge is stored beyond the pitch -- documented deviation, DESIGN.md.)
+            j = J.JPEGDEC(); assert j.openRAM(data); j.setArithMode(arith); j.setPixelType(pt); j.setCropArea(*crop)
+            cx, cy, cw, ch = j.getCropArea()
+            bypp = T.bpp_of(pt) // 8
+            fb = np.zeros((ch + 32) * cw * bypp, np.uint8); j.setFramebuffer(fb)
+            assert j.decode(0, 0, opt) == 1
+            got = fb[:ch * cw * bypp].reshape(ch, cw * bypp)
+            assert T.sha(got) == g["framebuffer"], (name, crop, pt, opt, "framebuffer")
+            j.close()

@@ -136,20 +136,46 @@ def test_delivery_schedule_equals_the_reference_callback_sequence():
     iWidthUsed, the JPEG_USES_DMA half) against the callback log of the compiled reference, WITHOUT a GPU: every fixture
     sampling x pixel type x scale x decode offset x setMaxOutputSize x crop -- including crop x scale, where the reference
     compares scaled MCU positions with the unscaled crop rectangle (SURVEY.md A.5: fewer rows at 1/2, no callbacks at 1/4
-    and 1/8); reproduced literally (src/jpeg.inl:5062-5084, :5111, :5135, :5300-5336)."""
-    from oracle import refdrv
-    if not refdrv.available("sse"):
-        pytest.skip("oracle/_ref not built here")
-    ref = refdrv.Ref("sse")
-    rng = np.random.default_rng(5)
+    and 1/8); reproduced literally (src/jpeg.inl:5062-5084, :5111, :5135, :5300-5336).  The reference's logs are recorded in
+    tests/golden/reference/host_schedule.json: per fixture, one "rc err calls digest" entry per case, in case order."""
+    want = T.reference_calls("host_schedule")
     checked = with_crop_scaled = 0
+    for name, cases in _schedule_cases():
+        assert len(cases) == len(want[name]), name
+        for (data, w, h, sub, crop, pt, opt, xo, yo, maxm), rec in zip(cases, want[name]):
+            rc, err, ncalls, digest = rec.split()
+            rc, err, ncalls = int(rc), int(err), int(ncalls)
+            assert rc in (0, 1)     # 0: the crop reaches below the image and the reference runs out of data
+            j2 = J.JPEGDEC()
+            assert j2.openRAM(data)
+            if crop is not None:
+                j2.setCropArea(*crop)
+            cx, cy, cw, ch = j2.getCropArea()
+            g = _Geom(w, h, cx, cy, cw, ch, xo, yo, sub, pt, opt, maxm if maxm else 1000)
+            got = _schedule(g)
+            if rc == 0:
+                assert err == J.JPEG_DECODE_ERROR and cy + ch > h
+                got = got[:ncalls]     # the calls made before the reference failed
+            assert len(got) == ncalls and T.log_sha(got) == digest, (name, crop, pt, opt, xo, yo, maxm, got[:3])
+            checked += 1
+            with_crop_scaled += int(crop is not None and (opt & 14) != 0)
+    assert checked > 1500 and with_crop_scaled > 300
+
+
+def _schedule_cases():
+    """[(fixture, [(data, w, h, subsampling, crop, pixel type, options, x offset, y offset, setMaxOutputSize)])]: every fixture
+    sampling x pixel type x scale x decode offset x setMaxOutputSize x crop, with four seeded random crops per fixture"""
+    rng = np.random.default_rng(5)
+    out = []
     for name in ("tulips", "zebra", "ncc1701", "sciopero", "lange", "croptest", "octocat_small"):
         data = T.image(name)
         j = J.JPEGDEC()
         assert j.openRAM(data)
         w, h, sub = j.getWidth(), j.getHeight(), j.getSubSample()
+        j.close()
         crops = [None, (50, 50, 125, 170), (96, 64, 256, 192), (0, 0, 64, 64), (16, 32, 100, 40)]
         crops += [(int(rng.integers(0, w)), int(rng.integers(0, h)), int(rng.integers(1, w)), int(rng.integers(1, h))) for _ in range(4)]
+        cases = []
         for crop in crops:
             if crop is not None and (crop[0] + 16 >= w or crop[1] + 16 >= h):
                 continue
@@ -158,30 +184,29 @@ def test_delivery_schedule_equals_the_reference_callback_sequence():
                     for (xo, yo, maxm) in ((0, 0, 0), (7, 3, 0), (0, 0, 3)):
                         if crop is not None and (xo or maxm) and opt:
                             continue
-                        rc, err, img, log = ref.decode_cb(data, pt, opt, xoff=xo, yoff=yo, crop=crop, max_mcus=maxm)
-                        assert rc in (0, 1)     # 0: the crop reaches below the image and the reference runs out of data
-                        j2 = J.JPEGDEC()
-                        assert j2.openRAM(data)
-                        if crop is not None:
-                            j2.setCropArea(*crop)
-                        cx, cy, cw, ch = j2.getCropArea()
-                        g = _Geom(w, h, cx, cy, cw, ch, xo, yo, sub, pt, opt, maxm if maxm else 1000)
-                        got = _schedule(g)
-                        want = [(r[0], r[1], r[2], r[3], r[4], r[6]) for r in log]
-                        if rc == 0:
-                            assert err == J.JPEG_DECODE_ERROR and cy + ch > h
-                            got = got[:len(want)]     # the calls made before the reference failed
-                        assert got == want, (name, crop, pt, opt, xo, yo, maxm, got[:3], want[:3])
-                        checked += 1
-                        with_crop_scaled += int(crop is not None and (opt & 14) != 0)
-        j.close()
-    assert checked > 1500 and with_crop_scaled > 300
+                        cases.append((data, w, h, sub, crop, pt, opt, xo, yo, maxm))
+        out.append((name, cases))
+    return out
+
+
+def record_schedule(refs):
+    out = {}
+    for name, cases in _schedule_cases():
+        out[name] = []
+        for data, w, h, sub, crop, pt, opt, xo, yo, maxm in cases:
+            rc, err, img, log = refs["sse"].decode_cb(data, pt, opt, xoff=xo, yoff=yo, crop=crop, max_mcus=maxm)
+            calls = [(r[0], r[1], r[2], r[3], r[4], r[6]) for r in log]
+            out[name].append("%d %d %d %s" % (rc, err, len(calls), T.log_sha(calls)))
+    return out
 
 
 def test_bench_reference_arm_line_has_the_contract_keys():
     """`bench.py --impl reference` (the reference's own CPU path on the host cores) needs no GPU: run one step here and check
-    the JSON line the driver parses."""
+    the JSON line it prints.  It times the reference itself, so it runs where build() could compile it into oracle/_ref."""
     import json, subprocess, sys
+    from oracle import refdrv
+    if not refdrv.available("sse"):
+        pytest.skip("the reference build oracle/_ref/libjpegdec_ref_sse.so is not present")
     r = subprocess.run([sys.executable, os.path.join(T.ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "0"],
                        stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=600)
     assert r.returncode == 0, r.stderr[-1500:]

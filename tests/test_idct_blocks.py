@@ -1,5 +1,5 @@
 """CPU tier: single 8x8 blocks through (a) the reference's own JPEGIDCT (static function, reachable inside
-oracle/ref_shim.c's TU), (b) the C restatement, (c) the per-thread code the CUDA kernel executes (tests/hostsim) --
+oracle/ref_shim.c's TU; its outputs recorded as digests in tests/golden/reference/idct_blocks.json), (b) the C restatement, (c) the per-thread code the CUDA kernel executes (tests/hostsim) --
 random sparse blocks including extreme coefficient x quant products that exercise the int16 wrap-around of the SSE2
 build and the two corner cases the kernel's unified column pass patches."""
 import ctypes as C
@@ -50,12 +50,23 @@ def _blocks(rng, n):
             yield coef, quant, fl
 
 
+def record_idct_blocks(refs):
+    """digest of the reference's JPEGIDCT output for every block of the test's seeded sequence, per arithmetic build"""
+    libs = [C.CDLL(os.path.join(T.ROOT, "oracle", "_ref", "libjpegdec_ref_%s.so" % m)) for m in ("sse", "scalar")]
+    outs = ([], [])
+    for coef, quant, fl in _blocks(np.random.default_rng(11), 12000):
+        for arith in (0, 1):
+            o_ref = np.zeros(64, np.uint8)
+            libs[arith].ref_idct(coef.ctypes.data, quant.ctypes.data, fl, 0, o_ref.ctypes.data)
+            outs[arith].append(o_ref)
+    return {"sse": T.sha(np.concatenate(outs[0])), "scalar": T.sha(np.concatenate(outs[1]))}
+
+
 def test_idct_blocks_reference_restatement_kernelcode():
-    from oracle import refdrv
     orc = T.oracle()
     sim = T.hostsim()
-    refs = [C.CDLL(os.path.join(T.ROOT, "oracle", "_ref", "libjpegdec_ref_%s.so" % m)) if refdrv.available(m) else None
-            for m in ("sse", "scalar")]
+    want = T.reference_calls("idct_blocks")
+    outs = ([], [])
     rng = np.random.default_rng(11)
     n = 0
     for coef, quant, fl in _blocks(rng, 12000):
@@ -70,9 +81,9 @@ def test_idct_blocks_reference_restatement_kernelcode():
                 sim.hostsim_idct_packed_general(coef.ctypes.data, quant.ctypes.data, fl, o_g.ctypes.data)
                 assert np.array_equal(o_or, o_p), ("packed", hex(fl))
                 assert np.array_equal(o_or, o_g), ("packed general", hex(fl))
-            if refs[arith] is not None:
-                o_ref = np.zeros(64, np.uint8)
-                refs[arith].ref_idct(coef.ctypes.data, quant.ctypes.data, fl, 0, o_ref.ctypes.data)
-                assert np.array_equal(o_ref, o_or), (arith, hex(fl))
+            outs[arith].append(o_or)
             n += 1
     assert n > 20000
+    # the restatement's blocks, in order, are the reference's (tests/golden/reference/idct_blocks.json)
+    assert T.sha(np.concatenate(outs[0])) == want["sse"]
+    assert T.sha(np.concatenate(outs[1])) == want["scalar"]

@@ -1,7 +1,8 @@
 """CPU tier: the checkers themselves.  (1) the C restatement (oracle/jpegdec_oracle.c) and the sequential
 stepper of the kernels' per-thread code (tests/hostsim) reproduce the digests the *compiled reference*
 produced for every bundled image x pixel type x scale x arithmetic build (tests/golden/digests.json, written
-by tests/golden/make_golden.py); (2) where oracle/_ref is present, they are compared with it live too."""
+by tests/golden/make_golden.py); (2) they reproduce what the compiled reference returned for dithered, synthetic and
+seeded random files (tests/golden/reference/, written by tests/golden/make_reference_golden.py)."""
 import numpy as np
 import pytest
 
@@ -57,49 +58,86 @@ def test_committed_golden_frame():
     assert rc == 1 and np.array_equal(out, want)
 
 
-@pytest.mark.parametrize("name", ["tulips", "zebra", "ncc1701", "lange"])
-def test_dither_restatement_vs_live_reference(name):
-    from oracle import refdrv
-    if not refdrv.available("sse"):
-        pytest.skip("oracle/_ref not built here")
-    data = T.image(name)
+DITHER_NAMES = ["tulips", "zebra", "ncc1701", "lange"]
+
+
+def _dither_cases(name):
+    """(key, mode, arith, pt, opt, width, height, bytes of a row that hold image pixels)"""
     inf = T.digests()[name]["info"]
     for mode, arith in MODES:
-        ref = refdrv.Ref(mode)
         for pt, ptn in T.DITHERS:
             for opt in (0, 2):
-                rc, err, img, log = ref.decode_dither(data, pt, opt)
-                rc2, out = T.oracle_decode(data, pt, opt, arith, inf["width"], inf["height"])
                 s = 1 if opt else 0
                 wb = ((((inf["width"] + (1 << s) - 1) >> s) * T.bpp_of(pt)) + 7) // 8
-                assert rc == rc2 == 1
-                assert np.array_equal(out[:img.shape[0], :wb], img[:, :wb]), (name, mode, ptn, opt)
+                yield "%s/%s/%s/%d" % (name, mode, ptn, opt), mode, arith, pt, opt, inf["width"], inf["height"], wb
 
 
-def test_synthetic_formats_vs_live_reference():
+def record_dither(refs):
+    out = {}
+    for name in DITHER_NAMES:
+        for key, mode, arith, pt, opt, w, h, wb in _dither_cases(name):
+            rc, err, img, log = refs[mode].decode_dither(T.image(name), pt, opt)
+            out[key] = {"rc": rc, "rows": img.shape[0], "sha": T.sha(img[:, :wb])}
+    return out
+
+
+@pytest.mark.parametrize("name", DITHER_NAMES)
+def test_dither_restatement_vs_live_reference(name):
+    want = T.reference_calls("oracle_dither")
+    data = T.image(name)
+    for key, mode, arith, pt, opt, w, h, wb in _dither_cases(name):
+        g = want[key]
+        rc2, out = T.oracle_decode(data, pt, opt, arith, w, h)
+        assert g["rc"] == rc2 == 1
+        assert T.sha(out[:g["rows"], :wb]) == g["sha"], key
+
+
+def _synthetic_format_cases():
     """4:2:2, 4:4:4, grayscale, no-restart odd-sized 4:2:0: bundled images do not cover them."""
-    from oracle import refdrv
     from tests import synth
-    if not refdrv.available("sse"):
-        pytest.skip("oracle/_ref not built here")
-    cases = {"gray": synth.synth_jpeg(320, 200, 1, 75, gray=True),
-             "s444": synth.synth_jpeg(173, 131, 2, 80, subsampling="4:4:4"),
-             "s422": synth.synth_jpeg(173, 131, 3, 80, subsampling="4:2:2"),
-             "odd420": synth.synth_jpeg(301, 203, 4, 90, restart_rows=0)}
+    return {"gray": (synth.synth_jpeg(320, 200, 1, 75, gray=True), 320, 200),
+            "s444": (synth.synth_jpeg(173, 131, 2, 80, subsampling="4:4:4"), 173, 131),
+            "s422": (synth.synth_jpeg(173, 131, 3, 80, subsampling="4:2:2"), 173, 131),
+            "odd420": (synth.synth_jpeg(301, 203, 4, 90, restart_rows=0), 301, 203)}
+
+
+def _synthetic_format_keys(cases):
     for mode, arith in MODES:
-        ref = refdrv.Ref(mode)
-        for n, data in cases.items():
-            rc0, inf = ref.info(data)
+        for n in cases:
             for pt, ptn in T.PTS:
                 if n == "gray" and pt == 2:
                     continue  # reference writes 16-bit pixels into a 32-bit buffer here (JPEGPutMCUGray): undefined
                 for opt, sn in T.SCALES:
-                    rc, err, img, _ = ref.decode_cb(data, pt, opt, want_log=False)
-                    rc1, o1 = T.oracle_decode(data, pt, opt, arith, inf.width, inf.height)
-                    rc2, o2, _ = T.hostsim_decode(data, pt, opt, arith, inf.width, inf.height)
-                    assert rc == rc1 == rc2 == 1
-                    assert np.array_equal(o1, img), (n, mode, ptn, sn)
-                    assert np.array_equal(o2, img), (n, mode, ptn, sn)
+                    yield "%s/%s/%s/%s" % (mode, n, ptn, sn), mode, arith, n, pt, opt
+
+
+def record_synthetic_formats(refs):
+    cases = _synthetic_format_cases()
+    out = {"input/" + n: {"input": T.sha(np.frombuffer(d, dtype=np.uint8))} for n, (d, w, h) in cases.items()}
+    for key, mode, arith, n, pt, opt in _synthetic_format_keys(cases):
+        data, w, h = cases[n]
+        rc0, inf = refs[mode].info(data)
+        assert (inf.width, inf.height) == (w, h)
+        rc, err, img, _ = refs[mode].decode_cb(data, pt, opt, want_log=False)
+        out[key] = {"rc": rc, "shape": list(img.shape), "sha": T.sha(img)}
+    return out
+
+
+def test_synthetic_formats_vs_live_reference():
+    """4:2:2, 4:4:4, grayscale, no-restart odd-sized 4:2:0: the C restatement and the kernel stepper against what the
+    compiled reference returned for the same files."""
+    want = T.reference_calls("oracle_synthetic")
+    cases = _synthetic_format_cases()
+    for n, (data, w, h) in cases.items():
+        T.check_input(want["input/" + n], data, n)
+    for key, mode, arith, n, pt, opt in _synthetic_format_keys(cases):
+        data, w, h = cases[n]
+        g = want[key]
+        rc1, o1 = T.oracle_decode(data, pt, opt, arith, w, h)
+        rc2, o2, _ = T.hostsim_decode(data, pt, opt, arith, w, h)
+        assert g["rc"] == rc1 == rc2 == 1
+        assert list(o1.shape) == g["shape"] and T.sha(o1) == g["sha"], key
+        assert list(o2.shape) == g["shape"] and T.sha(o2) == g["sha"], key
 
 
 @pytest.mark.parametrize("name", ["sciopero", "st_peters", "zebra", "octocat_small", "batman", "ncc1701", "lange"])
@@ -207,16 +245,11 @@ def test_progressive_dc_thumbnail_restatement_and_kernel_stepper(name):
                 assert rc == 1 and T.sha(sim) == g[key]["sha"], (name, key, "stepper")
 
 
-def test_seeded_random_sweep_vs_live_reference():
+def _seeded_sweep_cases():
     """120 seeded random files (size 8..260, quality 15..100, every sampling, gray, restart interval 0 / rows, baseline and
-    progressive): the C restatement and the kernel stepper against the compiled reference, random pixel type and scale."""
-    from oracle import refdrv
+    progressive), each with a random arithmetic build, pixel type and scale."""
     from tests import synth
-    if not refdrv.available("sse"):
-        pytest.skip("oracle/_ref not built here")
     rng = np.random.default_rng(20240923)
-    refs = {m: refdrv.Ref(m) for m, _ in MODES}
-    checked = 0
     for case in range(120):
         w, h = int(rng.integers(8, 261)), int(rng.integers(8, 261))
         q = int(rng.integers(15, 101))
@@ -231,13 +264,32 @@ def test_seeded_random_sweep_vs_live_reference():
             pts = [p for p in pts if p != 3]          # the reference crashes on progressive -> 8-bit gray
         pt = pts[int(rng.integers(0, len(pts)))]
         opt = 8 if prog else [0, 2, 4, 8][int(rng.integers(0, 4))]
+        yield case, data, w, h, (q, sub, gray, rr, prog), mode, arith, pt, opt
+
+
+def record_seeded_sweep(refs):
+    out = {}
+    for case, data, w, h, desc, mode, arith, pt, opt in _seeded_sweep_cases():
         rc, err, img, _ = refs[mode].decode_cb(data, pt, opt, want_log=False)
-        assert rc == 1, (case, w, h, q, sub, gray, rr, prog, err)
+        assert rc == 1, (case, w, h, desc, err)
+        out[str(case)] = {"input": T.sha(np.frombuffer(data, dtype=np.uint8)), "rc": rc, "shape": list(img.shape), "sha": T.sha(img)}
+    return out
+
+
+def test_seeded_random_sweep_vs_live_reference():
+    """The seeded random files of _seeded_sweep_cases: the C restatement and the kernel stepper against what the compiled
+    reference returned for them."""
+    want = T.reference_calls("oracle_sweep")
+    checked = 0
+    for case, data, w, h, desc, mode, arith, pt, opt in _seeded_sweep_cases():
+        g = want[str(case)]
+        T.check_input(g, data, case)
+        assert g["rc"] == 1
         rc1, o1 = T.oracle_decode(data, pt, opt, arith, w, h)
         rc2, o2, _ = T.hostsim_decode(data, pt, opt, arith, w, h)
         assert rc1 == 1 and rc2 == 1, (case, rc1, rc2)
-        assert np.array_equal(o1, img), ("restatement", case, w, h, q, sub, gray, rr, prog, mode, pt, opt)
-        assert np.array_equal(o2, img), ("stepper", case, w, h, q, sub, gray, rr, prog, mode, pt, opt)
+        assert list(o1.shape) == g["shape"] and T.sha(o1) == g["sha"], ("restatement", case, w, h, desc, mode, pt, opt)
+        assert list(o2.shape) == g["shape"] and T.sha(o2) == g["sha"], ("stepper", case, w, h, desc, mode, pt, opt)
         checked += 1
     assert checked == 120
 
